@@ -1,12 +1,16 @@
 """bench.py -- headline metric of BASELINE.json: video frames/s through tokenize + decode_from_code_indices,
 17x128x128 clips, bf16, README config (BASELINE.json configs[1]), data-parallel over N GPUs of one node.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
          bench.py --gpus N --steps K --warmup W
 
 A "step" is one pass of the hot path over one batch of 4 synthetic clips per GPU (weak scaling: the batch
 is sharded by clip, no data-path collective in eval -- SURVEY.md 8e).  Prints ONE JSON line (rank 0).
+
+--dump-outputs DIR writes what the last timed step returned (rank 0) as DIR/codes.npy (float64, exact code indices)
+and DIR/recon.npy (float32).  Weights and inputs are seeded, so two builds run with the same arguments can be
+compared output for output.
 
 --impl reference times the reference's own CPU implementation of the path: the reference is pure Python and
 cannot travel to the GPU box, so this arm runs the restated oracle (oracle/restated.py, pinned bit-for-bit to
@@ -164,6 +168,25 @@ def _cpu_oracles():
             "bf16": OracleTokenizer(sd, dtype=torch.bfloat16, **README_KW)}
 
 
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, codes, recon):
+    """The arrays a caller of the timed path receives, as .npy files of at most DUMP_MAX_BYTES in all (the largest
+    workload writes 40 MB).  A reconstruction that does not fit is replaced by a fixed, seeded sample of its elements:
+    a 1-D array of the values at sorted flat indices, the same indices for the same shape."""
+    import numpy as np
+    arrays = {"codes": codes.detach().cpu().double().numpy(), "recon": recon.detach().float().cpu().numpy()}
+    if sum(a.nbytes for a in arrays.values()) > DUMP_MAX_BYTES:
+        r = arrays["recon"]
+        keep = (DUMP_MAX_BYTES - arrays["codes"].nbytes) // r.itemsize
+        idx = np.sort(np.random.default_rng(0).choice(r.size, size=keep, replace=False))
+        arrays["recon"] = r.reshape(-1)[idx]
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
+
+
 def _cpu_time_step(orc, video):
     t0 = time.perf_counter()
     orc.decode_from_code_indices(orc.tokenize(video))
@@ -185,7 +208,10 @@ def _cpu_pick_dtype(orcs, video1):
 def run_reference_arm(args):
     """CPU baseline: the reference's torch-eager CPU path (restated oracle), all host threads, bounded sample:
     fp32 or bf16 storage (whichever these host cores run faster), 4 clips per step like the GPU arm when the
-    K + W passes fit in ~3 minutes, else 1 clip (and a 5-frame clip if even that does not fit)."""
+    K + W passes fit in ~3 minutes, else 1 clip (and a 5-frame clip if even that does not fit).
+    With --dump-outputs the sample is fixed instead (fp32, one 17-frame clip), so that the dumped arrays do not depend
+    on the speed of the host.  CPU kernels still differ between instruction sets, so dumps from different hosts agree
+    to fp32 round-off, not bit for bit."""
     import torch
     import synth_data as Wt
 
@@ -194,14 +220,19 @@ def run_reference_arm(args):
         return
     cores = _best_cpu_threads()
     orcs = _cpu_oracles()
-    dt_name, secs = _cpu_pick_dtype(orcs, Wt.synth_video(1, 3, FRAMES, 128, seed=1))
+    frames = FRAMES
+    if args.dump_outputs:
+        dt_name, secs, sample_clips = "f32", {}, 1
+    else:
+        dt_name, secs = _cpu_pick_dtype(orcs, Wt.synth_video(1, 3, FRAMES, 128, seed=1))
+        passes = args.steps + max(args.warmup, 0)
+        sample_clips = CLIPS_PER_GPU
+        if secs[dt_name] * sample_clips * passes > 180.0:
+            sample_clips = 1
+        if secs[dt_name] * sample_clips * passes > 180.0:
+            frames = 5
     orc = orcs[dt_name]
-    passes = args.steps + max(args.warmup, 0)
-    frames, sample_clips = FRAMES, CLIPS_PER_GPU
-    if secs[dt_name] * sample_clips * passes > 180.0:
-        sample_clips = 1
-    if secs[dt_name] * sample_clips * passes > 180.0:
-        frames = 5
+
     def mk(nclips):
         v = Wt.synth_video(nclips, 3, frames, 128, seed=1)
         return v.to(torch.bfloat16) if dt_name == "bf16" else v
@@ -214,9 +245,13 @@ def run_reference_arm(args):
         _cpu_time_step(orc, video)
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        _cpu_time_step(orc, video)
+        codes = orc.tokenize(video)
+        recon = orc.decode_from_code_indices(codes)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, codes, recon)
     fps = sample_clips * frames * args.steps / dt
+    probe = "1-clip probe: " + ", ".join(f"{k} {v:.2f} s" for k, v in secs.items()) if secs else "fixed for --dump-outputs"
     out = {
         "impl": "reference", "metric": METRIC, "value": fps, "unit": "frames/s", "n_gpus": args.gpus,
         "steps": args.steps, "warmup": args.warmup, "ms_per_step": 1e3 * dt / args.steps,
@@ -224,9 +259,8 @@ def run_reference_arm(args):
         "config": {"workload": "README VideoTokenizer (BASELINE configs[1]), tokenize+decode, CPU torch eager",
                    "clips_per_step": sample_clips},
         "cpu_baseline": {"value": fps, "unit": "frames/s", "cores": cores, "kind": "port",
-                         "sample": f"{sample_clips} clip(s) ({frames}x128x128) per step, {dt_name} (1-clip probe: "
-                                   + ", ".join(f"{k} {v:.2f} s" for k, v in secs.items()) +
-                                   f"), {cores} threads, oracle/restated.py (torch CPU eager, same ATen ops the reference dispatches)"},
+                         "sample": f"{sample_clips} clip(s) ({frames}x128x128) per step, {dt_name} ({probe}), "
+                                   f"{cores} threads, oracle/restated.py (torch CPU eager, same ATen ops the reference dispatches)"},
         "e2e": {"value": fps, "unit": "frames/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
         "gpu_launches": 0,
     }
@@ -259,18 +293,25 @@ def cpu_baseline_sample():
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=400)     # ~3 s timed region: long enough to reach the power-limited clocks
-    ap.add_argument("--warmup", type=int, default=5)
+    # default: 400 timed steps (~3 s, long enough to reach the power-limited clocks), 3 for the CPU arm
+    ap.add_argument("--steps", type=int, default=None)
+    ap.add_argument("--warmup", type=int, default=None)     # default: 5, 1 for the CPU arm
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--workload", default="readme", choices=sorted(WORKLOADS))
     # consecutive steps (independent batches) are issued round-robin on this many CUDA streams, each replaying its own
     # CUDA-graph instances (magvit2_pytorch_b200.StreamLanes); 1 = strictly serial steps
     ap.add_argument("--lanes", type=int, default=int(os.environ.get("MV2_LANES", "3")))
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None)
     args = ap.parse_args()
-    if args.impl == "reference":
-        if args.steps == 400 and args.warmup == 5:
-            args.steps, args.warmup = 3, 1
+    cpu_arm = args.impl == "reference"
+    if args.steps is None:
+        args.steps = 3 if cpu_arm else 400
+    if args.warmup is None:
+        args.warmup = 1 if cpu_arm else 5
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if cpu_arm:
         run_reference_arm(args)
         return
 
@@ -341,13 +382,16 @@ def main():
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for i in range(args.steps):
-        lanes.run(step, dev_batches[i % NB])
+        last, _ = lanes.run(step, dev_batches[i % NB])
     lanes.join()                         # the timing stream waits for every lane: all K steps end inside the timed region
     e1.record()
     barrier()
     ms = e0.elapsed_time(e1)
     launches = eng.launches - l0
     clocks = clk.stop() if rank == 0 else None
+    if rank == 0 and args.dump_outputs:
+        # copied before any later call: with CUDA graphs the results live in the lane's static output buffers
+        dump_outputs(args.dump_outputs, *last)
     t = torch.tensor([ms], device=dev)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)

@@ -43,9 +43,10 @@ CONFIGS = {
     "mini_fsq": dict(kwargs=dict(image_size=32, init_dim=16, max_dim=64, use_fsq=True, fsq_levels=[8, 5, 5, 5],
                                  layers=README_LAYERS),
                      video=(2, 3, 9, 32, 32), wseed=0, vseed=1234, full=True),
-    # BASELINE.json configs[1] (README), one clip
+    # BASELINE.json configs[1] (README), one clip.  Tap channel stride 32 (readme / readme_bf16 and cfg4 / cfg4_bf16) keeps
+    # each fixture under 1 MB; an fp32 golden and its bf16 twin must use the same strides
     "readme": dict(kwargs=dict(image_size=128, init_dim=64, max_dim=512, codebook_size=1024, layers=README_LAYERS),
-                   video=(1, 3, 17, 128, 128), wseed=0, vseed=1234, full=False, cs=16, ss=8),
+                   video=(1, 3, 17, 128, 128), wseed=0, vseed=1234, full=False, cs=32, ss=8),
     # SURVEY 8f N1: the one conditioned layer type that runs in the reference (cond_residual = ResidualUnitMod /
     # Conv3DMod, M:680-753, M:946-988).  Conditioned layers must be the trailing ones (has_cond is never reset, M:1153).
     "mini_cond": dict(kwargs=dict(image_size=32, init_dim=16, max_dim=64, codebook_size=1024, dim_cond=12,
@@ -56,15 +57,15 @@ CONFIGS = {
     #     reference's OWN bf16 deviation from fp32, layer by layer.  Decode is run on the fp32 golden's codes ("identical
     #     codes fed to both sides"); the tokenize side stores the bf16 reference's own codes / pre-sign values.
     "readme_bf16": dict(kwargs=dict(image_size=128, init_dim=64, max_dim=512, codebook_size=1024, layers=README_LAYERS),
-                        video=(1, 3, 17, 128, 128), wseed=0, vseed=1234, full=False, cs=16, ss=8, dtype="bf16",
+                        video=(1, 3, 17, 128, 128), wseed=0, vseed=1234, full=False, cs=32, ss=8, dtype="bf16",
                         codes_from="readme"),
     "mini_bf16": dict(kwargs=dict(image_size=32, init_dim=16, max_dim=64, codebook_size=1024, layers=README_LAYERS),
                       video=(2, 3, 9, 32, 32), wseed=0, vseed=1234, full=True, dtype="bf16", codes_from="mini"),
     # BASELINE.json configs[3]: image 256, max_dim 1024 (attention-heavy: space-attention seq 1024, linear-attention seq 4096)
     "cfg4": dict(kwargs=dict(image_size=256, init_dim=64, max_dim=1024, codebook_size=1024, layers=README_LAYERS),
-                 video=(1, 3, 17, 256, 256), wseed=0, vseed=1234, full=False, cs=16, ss=16, rs=8),
+                 video=(1, 3, 17, 256, 256), wseed=0, vseed=1234, full=False, cs=32, ss=16, rs=8),
     "cfg4_bf16": dict(kwargs=dict(image_size=256, init_dim=64, max_dim=1024, codebook_size=1024, layers=README_LAYERS),
-                      video=(1, 3, 17, 256, 256), wseed=0, vseed=1234, full=False, cs=16, ss=16, rs=8, dtype="bf16",
+                      video=(1, 3, 17, 256, 256), wseed=0, vseed=1234, full=False, cs=32, ss=16, rs=8, dtype="bf16",
                       codes_from="cfg4"),
     # BASELINE.json configs[4]: FSQ variant of the README config, levels [8,5,5,5] (SURVEY 8d)
     "fsq": dict(kwargs=dict(image_size=128, init_dim=64, max_dim=512, use_fsq=True, fsq_levels=[8, 5, 5, 5], layers=README_LAYERS),

@@ -45,7 +45,9 @@ def _worker(rank, world, port, q):
         return avg
 
     ps, be, cm, aux, avg = lfq_train_losses(local, 10, world_reduce=reduce)
-    q.put((rank, ps.item(), be.item(), cm.item(), aux.item(), avg))
+    # a tensor would travel as a shared-memory handle that the parent can only open while this process is alive;
+    # a numpy array is pickled by value
+    q.put((rank, ps.item(), be.item(), cm.item(), aux.item(), avg.numpy()))
     dist.barrier()
     dist.destroy_process_group()
 
@@ -68,6 +70,7 @@ def test_lfq_batch_entropy_allreduce_world2_gloo():
     # batch entropy comes from the GLOBAL mean code probability -> identical on both ranks and equal to the
     # single-process value on the whole batch; per-sample entropy / commitment are per-rank means
     for rank, ps, be, cm, aux, avg in res:
+        avg = torch.from_numpy(avg)
         assert abs(be - be_all.item()) < 1e-5
         assert torch.allclose(avg, avg_all, atol=1e-6)
         assert abs(be - entropy_from_avg_prob(avg).item()) < 1e-6

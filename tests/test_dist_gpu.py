@@ -39,7 +39,10 @@ def _worker(rank, world, port, q, dtype_name):
         codes, recon = model(local, return_codes=True, return_recon=True)
         ps, be, cm = model.quantizer_loss_breakdown
         torch.cuda.synchronize()
-    q.put((rank, codes.cpu(), recon.float().cpu(), ps.item(), be.item(), cm.item(), model.quantizer_aux_loss.item()))
+    # numpy arrays are pickled by value; a tensor would travel as a shared-memory handle that the parent can only open
+    # while this process is alive
+    q.put((rank, codes.cpu().numpy(), recon.float().cpu().numpy(), ps.item(), be.item(), cm.item(),
+           model.quantizer_aux_loss.item()))
     dist.barrier()
     dist.destroy_process_group()
 
@@ -62,8 +65,8 @@ def test_train_mode_forward_world2_nccl(dtype_name):
         p.join(timeout=120)
         assert p.exitcode == 0
     g = load_golden("mini")
-    codes = torch.cat([r[1] for r in res])
-    recon = torch.cat([r[2] for r in res])
+    codes = torch.cat([torch.from_numpy(r[1]) for r in res])
+    recon = torch.cat([torch.from_numpy(r[2]) for r in res])
     cpu_model = build_product(g["kwargs"], g["wseed"])
     orc = build_oracle(cpu_model, g["kwargs"])
     ref_codes, pre = orc.tokenize(golden_video(g), return_presign=True)
