@@ -145,6 +145,24 @@ def pack_conv_in_kwpack(weight, bias, cpack=32):
     return pk
 
 
+def stage_modules(st, mod, decoder: bool) -> dict:
+    """Where a stage's parameters sit inside its layer module `mod` (the reference's nesting, M:1138-1318), by role.  Read by
+    Engine.prepare, which packs them, and by the training path, which differentiates them."""
+    if st.kind == "residual":       # Residual(Sequential(CausalConv3d, ELU, Conv3d 1x1x1, ELU, SqueezeExcite)) (M:930-944)
+        return dict(units=[dict(conv3=ru.fn[0].conv, conv1=ru.fn[2], se=ru.fn[4]) for ru in (list(mod) if st.nested else [mod])])
+    if st.kind == "cond_residual":
+        return dict(unit=mod)
+    if st.kind in ("compress_space", "compress_time"):
+        return dict(conv=mod.net[0] if decoder else mod.conv)
+    if st.kind in ("attend_space", "linear_attend_space"):      # Residual(attention), Residual(FeedForward)
+        return dict(attn=mod[0].fn, ff=mod[1].fn)
+    if st.kind == "attend_time":                               # Residual(TokenShift(...)) for both blocks
+        return dict(attn=mod[0].fn.fn, ff=mod[1].fn.fn)
+    if st.kind == "gateloop_time":                             # ToTimeSequence(Residual(SimpleGateLoopLayer))
+        return dict(gateloop=mod.fn.fn)
+    raise ValueError(st.kind)
+
+
 class Engine:
     """Executes the inference path of one VideoTokenizer on its parameters' device/dtype."""
 
@@ -206,13 +224,12 @@ class Engine:
         def f32(t):
             return t.detach().float().contiguous()
 
-        def pack_ru(ru, key):
-            seq = ru.fn
-            se = seq[4]
-            C_ = seq[2].weight.shape[0]
+        def pack_ru(u, key):
+            se, c1 = u["se"], u["conv1"]
+            C_ = c1.weight.shape[0]
             P[key] = dict(
-                conv3=pack_conv(seq[0].conv.weight, seq[0].conv.bias, dt),
-                conv1=pack_conv(seq[2].weight, seq[2].bias, dt),
+                conv3=pack_conv(u["conv3"].weight, u["conv3"].bias, dt),
+                conv1=pack_conv(c1.weight, c1.bias, dt),
                 wk=f32(se.to_k.weight.reshape(-1)), bk=float(se.to_k.bias.detach().float().item()),
                 w1=f32(se.net[0].weight.reshape(se.net[0].weight.shape[0], C_)), b1=f32(se.net[0].bias),
                 w2=f32(se.net[2].weight.reshape(C_, -1)), b2=f32(se.net[2].bias),
@@ -240,43 +257,43 @@ class Engine:
                           heads=la.heads, dim_head=la.dim_head)
 
         for side, layers in (("enc", m.encoder_layers), ("dec", m.decoder_layers)):
-            stages = m.stages if side == "enc" else list(reversed(m.stages))
+            decoder = side == "dec"
+            stages = m.stages if not decoder else list(reversed(m.stages))
             for i, st in enumerate(stages):
-                mod = layers[i]
+                parts = stage_modules(st, layers[i], decoder)
                 key = f"{side}{i}"
                 if st.kind == "residual":
-                    units = list(mod) if st.nested else [mod]
-                    for j, ru in enumerate(units):
-                        pack_ru(ru, f"{key}.{j}")
+                    for j, u in enumerate(parts["units"]):
+                        pack_ru(u, f"{key}.{j}")
                 elif st.kind == "cond_residual":
+                    mod = parts["unit"]
                     w = mod.conv.weights
                     wq = w.detach().to(dt).float()                  # the weights as the module holds them in this dtype
                     P[key] = dict(conv3=pack_conv(w, None, dt), conv1=pack_conv(mod.conv_out.weight, mod.conv_out.bias, dt),
                                   S=(wq * wq).sum(dim=(2, 3, 4)).contiguous(), eps=float(mod.conv.eps),
                                   wc=f32(mod.to_cond.weight), bc=f32(mod.to_cond.bias))
                 elif st.kind == "compress_space":
-                    if side == "enc":
-                        P[key] = pack_conv(mod.conv.weight, mod.conv.bias, dt)                     # (Co,Ci,3,3) -> k=(1,3,3)
+                    conv = parts["conv"]
+                    if not decoder:
+                        P[key] = pack_conv(conv.weight, conv.bias, dt)                 # (Co,Ci,3,3) -> k=(1,3,3)
                         if dt == torch.bfloat16:
-                            pack_conv_down_space(P[key], mod.conv.weight)
+                            pack_conv_down_space(P[key], conv.weight)
                     else:
-                        P[key] = pack_conv(mod.net[0].weight, mod.net[0].bias, dt, shuffle_q=4)    # (4Co,Ci,1,1)
+                        P[key] = pack_conv(conv.weight, conv.bias, dt, shuffle_q=4)    # (4Co,Ci,1,1)
                 elif st.kind == "compress_time":
-                    if side == "enc":
-                        P[key] = pack_conv(mod.conv.weight, mod.conv.bias, dt, k=(3, 1, 1))        # Conv1d (Co,Ci,3)
+                    conv = parts["conv"]
+                    if not decoder:
+                        P[key] = pack_conv(conv.weight, conv.bias, dt, k=(3, 1, 1))             # Conv1d (Co,Ci,3)
                     else:
-                        P[key] = pack_conv(mod.net[0].weight, mod.net[0].bias, dt, k=(1, 1, 1), shuffle_q=2)  # Conv1d (2Co,Ci,1)
-                elif st.kind == "attend_space":
-                    pack_attn(mod[0].fn, key + ".attn")
-                    pack_ffn(mod[1].fn, key + ".ff")
-                elif st.kind == "attend_time":
-                    pack_attn(mod[0].fn.fn, key + ".attn")
-                    pack_ffn(mod[1].fn.fn, key + ".ff")
+                        P[key] = pack_conv(conv.weight, conv.bias, dt, k=(1, 1, 1), shuffle_q=2)  # Conv1d (2Co,Ci,1)
+                elif st.kind in ("attend_space", "attend_time"):
+                    pack_attn(parts["attn"], key + ".attn")
+                    pack_ffn(parts["ff"], key + ".ff")
                 elif st.kind == "linear_attend_space":
-                    pack_lin(mod[0].fn, key + ".attn")
-                    pack_ffn(mod[1].fn, key + ".ff")
+                    pack_lin(parts["attn"], key + ".attn")
+                    pack_ffn(parts["ff"], key + ".ff")
                 elif st.kind == "gateloop_time":
-                    gl = mod.fn.fn
+                    gl = parts["gateloop"]
                     P[key] = dict(gamma=f32(gl.norm.gamma), qkva=pack_conv(gl.to_qkva[0].weight[:, :, None, None, None], None, dt))
         if m.has_cond:
             for side, stem in (("enc", m.encoder_cond_in), ("dec", m.decoder_cond_in)):
@@ -295,6 +312,21 @@ class Engine:
 
     def _new(self, shape, dtype=None):
         return torch.empty(shape, device=self.device, dtype=dtype or self.dtype)
+
+    def _tc_launch(self, entry, args, kind, k, out, macs, **shape):
+        """Launches the tcgen05 conv entry point `entry` (kind "slab" | "tap") on an output of `out` = (B, T, H, W) positions.
+        Under profile_convs CUDA events bracket the launch; when conv_log is set, the launch's shape is recorded there."""
+        if self._prof is not None:
+            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+            e0.record()
+        check(getattr(self.lib, entry)(C.byref(args), self._stream()), entry)
+        if self._prof is not None:
+            e1.record()
+            self._prof.append((e0, e1, 2.0 * out[0] * out[1] * out[2] * out[3] * macs, kind, k[0] * k[1] * k[2]))
+        if self.conv_log is not None:
+            self.conv_log.append(dict(kind=kind, k=tuple(k), out=out, **shape))
+        self.tc_calls += 1
+        self.slab_calls += int(kind == "slab")
 
     def conv(self, x, pk: ConvPack, *, stride=(1, 1, 1), pad=None, out_spatial=None, act=ACT_NONE,
              res=None, shuffle=SHUFFLE_NONE, token_shift=False, out_cf=False, oscale=None):
@@ -337,26 +369,10 @@ class Engine:
                 ta.w = _ptr(pk.w_down)
                 use_slab = True
             if use_slab or self.lib.mv2_tc_conv_supported(C.byref(ta)):
-                if self._prof is not None:
-                    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-                    e0.record()
-                if use_down:
-                    check(self.lib.mv2_tc_down_space_forward(C.byref(ta), self._stream()), "mv2_tc_down_space_forward")
-                    self.slab_calls += 1
-                elif use_slab:
-                    check(self.lib.mv2_tc_slab_forward(C.byref(ta), self._stream()), "mv2_tc_slab_forward")
-                    self.slab_calls += 1
-                else:
-                    check(self.lib.mv2_tc_conv_forward(C.byref(ta), self._stream()), "mv2_tc_conv_forward")
-                if self._prof is not None:
-                    e1.record()
-                    self._prof.append((e0, e1, 2.0 * B * To * Ho * Wo * pk.macs,
-                                       "slab" if use_slab else "tap", pk.k[1] * pk.k[2] * pk.k[0]))
-                if self.conv_log is not None:
-                    self.conv_log.append(dict(kind="slab" if use_slab else "tap", Ci=Ci, Co=co_out, k=tuple(pk.k), out=(B, To, Ho, Wo),
-                                              geglu=pk.epi_mode == 1, shuffle=shuffle, res=res is not None))
+                entry = "mv2_tc_down_space_forward" if use_down else "mv2_tc_slab_forward" if use_slab else "mv2_tc_conv_forward"
+                self._tc_launch(entry, ta, "slab" if use_slab else "tap", pk.k, (B, To, Ho, Wo), pk.macs, Ci=Ci, Co=co_out,
+                                geglu=pk.epi_mode == 1, shuffle=shuffle, res=res is not None)
                 self.launches += 1
-                self.tc_calls += 1
                 return y
             assert not out_cf, "channels-first output is a tcgen05 slab-kernel feature"
             assert pk.w is not None and pk.epi_mode == 0 and Ci == pk.Ci, "tcgen05-only weight pack has no CUDA-core fallback"
@@ -386,7 +402,6 @@ class Engine:
         B, T, H, W, Cc = x.shape
         F_, Pn = B * T, H * W
         st = self._stream()
-        dt = _dt(self.dtype)
         c3, c1 = p["conv3"], p["conv1"]
         if self.dtype == torch.bfloat16 and self.use_tc and self.fuse_ru and c3.w_tc is not None and self.tc_variant != "tap":
             ra = TcRuArgs(x=_ptr(x), w3=_ptr(c3.w_tc), b3=_ptr(c3.bias_tc), w1=_ptr(c1.w_tc), b1=_ptr(c1.bias_tc),
@@ -397,36 +412,37 @@ class Engine:
                 ws = self._new((self.lib.mv2_tc_ru_workspace_bytes(C.byref(ra)) // 4,), torch.float32)
                 ra.y, ra.se_ws = _ptr(y), _ptr(ws)
                 nrec = self.lib.mv2_tc_ru_records(C.byref(ra))
-                if self._prof is not None:
-                    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-                    e0.record()
-                check(self.lib.mv2_tc_ru_forward(C.byref(ra), st), "mv2_tc_ru_forward")
-                if self._prof is not None:
-                    e1.record()
-                    self._prof.append((e0, e1, 2.0 * B * T * H * W * (c3.macs + c1.macs), "slab", c3.k[0] * c3.k[1] * c3.k[2]))
-                if self.conv_log is not None:
-                    self.conv_log.append(dict(kind="slab", Ci=Cc, Co=Cc, k=tuple(c3.k), out=(B, T, H, W), geglu=False, shuffle=0,
-                                              res=False, fused_ru=True))
+                self._tc_launch("mv2_tc_ru_forward", ra, "slab", c3.k, (B, T, H, W), c3.macs + c1.macs, Ci=Cc, Co=Cc, geglu=False,
+                                shuffle=0, res=False, fused_ru=True)
                 gates = self._new((F_, Cc), torch.float32)
                 check(self.lib.mv2_se_gate_records(_ptr(ws), nrec, F_, Cc, p["hidden"], _ptr(p["w1"]), _ptr(p["b1"]), _ptr(p["w2"]),
                                                    _ptr(p["b2"]), _ptr(gates), st), "mv2_se_gate_records")
                 out = self._new(x.shape)
-                check(self.lib.mv2_gate_residual(_ptr(y), _ptr(x), _ptr(gates), _ptr(out), dt, F_, Pn, Cc, st), "mv2_gate_residual")
+                check(self.lib.mv2_gate_residual(_ptr(y), _ptr(x), _ptr(gates), _ptr(out), _dt(self.dtype), F_, Pn, Cc, st),
+                      "mv2_gate_residual")
                 self.launches += 4
-                self.tc_calls += 1
-                self.slab_calls += 1
                 self.fused_ru_calls += 1
                 return out
+        if not (self.dtype == torch.bfloat16 and self.se_tail and "w1b" in p
+                and self.lib.mv2_se_tail_supported(F_, Pn, Cc, p["hidden"])):
+            return self.residual_unit_unfused(x, p)[0]
         h = self.conv(x, c3, act=ACT_ELU)
         y = self.conv(h, c1, act=ACT_ELU)
-        if (self.dtype == torch.bfloat16 and self.se_tail and "w1b" in p
-                and self.lib.mv2_se_tail_supported(F_, Pn, Cc, p["hidden"])):
-            out = self._new(x.shape)
-            check(self.lib.mv2_se_tail(_ptr(y), _ptr(x), _ptr(out), F_, Pn, Cc, p["hidden"], _ptr(p["wk"]), p["bk"],
-                                       _ptr(p["w1b"]), _ptr(p["b1"]), _ptr(p["w2b"]), _ptr(p["b2"]), st), "mv2_se_tail")
-            self.launches += 1
-            self.se_tail_calls += 1
-            return out
+        out = self._new(x.shape)
+        check(self.lib.mv2_se_tail(_ptr(y), _ptr(x), _ptr(out), F_, Pn, Cc, p["hidden"], _ptr(p["wk"]), p["bk"],
+                                   _ptr(p["w1b"]), _ptr(p["b1"]), _ptr(p["w2b"]), _ptr(p["b2"]), st), "mv2_se_tail")
+        self.launches += 1
+        self.se_tail_calls += 1
+        return out
+
+    def residual_unit_unfused(self, x, p):
+        """ResidualUnit on separate launches: h = ELU(conv3(x)), y = ELU(conv1(h)), SE pool, gate MLP, gate + residual.
+        Returns (out, h, y); the training backward differentiates through the intermediate h and y."""
+        B, T, H, W, Cc = x.shape
+        F_, Pn = B * T, H * W
+        st, dt = self._stream(), _dt(self.dtype)
+        h = self.conv(x, p["conv3"], act=ACT_ELU)
+        y = self.conv(h, p["conv1"], act=ACT_ELU)
         ws = self._new((self.lib.mv2_se_workspace_bytes(F_, Pn, Cc) // 4,), torch.float32)
         gates = self._new((F_, Cc), torch.float32)
         check(self.lib.mv2_se_pool(_ptr(y), dt, F_, Pn, Cc, _ptr(p["wk"]), p["bk"], _ptr(ws), st), "mv2_se_pool")
@@ -435,7 +451,7 @@ class Engine:
         out = self._new(x.shape)
         check(self.lib.mv2_gate_residual(_ptr(y), _ptr(x), _ptr(gates), _ptr(out), dt, F_, Pn, Cc, st), "mv2_gate_residual")
         self.launches += 3
-        return out
+        return out, h, y
 
     def dense_small(self, x, w, b, act=ACT_NONE):
         """fp32 y[b][n] = act(x[b] . w[n] + bias[n]) (cond stems M:1344-1352, to_cond M:983)."""
@@ -682,12 +698,15 @@ class Engine:
         return out[0]
 
     # ------------------------------------------------------------------ the path
-    def encode_cl(self, video: torch.Tensor, first_frame: bool = True, cond=None):
-        """video (B,C,T,H,W) on device -> encoder output, channels-last.  Reference encode M:1523-1576; the time_padding
-        zero frames are only prepended when the clip starts with a first frame (video_contains_first_frame, M:1534-1537)."""
+    def conv_in_cl(self, video: torch.Tensor, first_frame: bool = True):
+        """conv_in (M:1109) of video (B,C,T,H,W) -> (channels-last feature map, saved).  The time_padding zero frames are only
+        prepended when the clip starts with a first frame (video_contains_first_frame, M:1534-1537).  `saved` holds the
+        channels-last inputs of the causal conv that a weight gradient needs: "rest_in" (frames 1.., first frame encoded
+        separately) or "padded_in" (the zero-prepended clip, pad_mode != 'constant')."""
         m = self.model
         t_pad = m.time_padding if first_frame else 0
         pin = self._packs.get("conv_in_tc")
+        saved = {}
         if m.separate_first_frame_encoding and first_frame:
             # M:1553-1561: the first frame goes through its own 2-D conv, frames 1.. through the causal conv_in on their own,
             # then the feature map is [time_padding zero frames, first, rest]
@@ -695,18 +714,54 @@ class Engine:
             v_cl = self.to_channels_last(video, 0)
             parts = [(self.conv(self.copy_frames(v_cl, 0, 1), self._packs["conv_in_ff"]), t_pad)]
             if T > 1:
-                parts.append((self.causal_conv_padded(self.copy_frames(v_cl, 1, T - 1), self._packs["conv_in"], m.conv_in.pad_mode), t_pad + 1))
+                saved["rest_in"] = self.copy_frames(v_cl, 1, T - 1)
+                parts.append((self.causal_conv_padded(saved["rest_in"], self._packs["conv_in"], m.conv_in.pad_mode), t_pad + 1))
             x = self._new((B, T + t_pad, H, W, parts[0][0].shape[-1]))
             for i, (part, t0) in enumerate(parts):
                 self.copy_frames(part, 0, part.shape[1], dst=x, dst_t0=t0, zero_front=(i == 0))
         elif m.conv_in.pad_mode != "constant":
-            x = self.causal_conv_padded(self.to_channels_last(video, t_pad), self._packs["conv_in"], m.conv_in.pad_mode)
+            saved["padded_in"] = self.to_channels_last(video, t_pad)
+            x = self.causal_conv_padded(saved["padded_in"], self._packs["conv_in"], m.conv_in.pad_mode)
         elif self.dtype == torch.bfloat16 and self.use_tc and pin is not None:
             x = self.ingest_kwpack(video, t_pad, pin)
             x = self.conv(x, pin, pad=(pin.k_tc[0] - 1, pin.k_tc[1] // 2, 0))
         else:
             x = self.to_channels_last(video, t_pad)
             x = self.conv(x, self._packs["conv_in"])
+        return x, saved
+
+    def conv_out_cf(self, x: torch.Tensor, first_frame: bool = True):
+        """conv_out (M:1127) of the decoder output x (B,T,H,W,C) -> (video (B,3,T,H,W), saved).  The leading time_padding
+        frames are dropped only for clips that contain a first frame (M:1646-1647).  `saved` holds "rest_out", the frames
+        the causal conv read when the first frame is decoded separately."""
+        m = self.model
+        pk = self._packs["conv_out"]
+        B, T, H, W, Cc = x.shape
+        tp = m.time_padding if first_frame else 0
+        saved = {}
+        if m.separate_first_frame_encoding and first_frame:
+            # M:1633-1639: conv_out_first_frame on frame `tp`, the causal conv_out on the frames after it, re-attached
+            first = self.conv(self.copy_frames(x, tp, 1), self._packs["conv_out_ff"])
+            out = self._new((B, T - tp, H, W, first.shape[-1]))
+            self.copy_frames(first, 0, 1, dst=out, dst_t0=0)
+            if T - tp > 1:
+                saved["rest_out"] = self.copy_frames(x, tp + 1, T - tp - 1)
+                rest = self.causal_conv_padded(saved["rest_out"], pk, m.conv_out.pad_mode)
+                self.copy_frames(rest, 0, T - tp - 1, dst=out, dst_t0=1)
+            return self.to_channels_first(out), saved
+        if m.conv_out.pad_mode != "constant":
+            return self.to_channels_first(self.causal_conv_padded(x, pk, m.conv_out.pad_mode), t_crop=tp), saved
+        if (self.dtype == torch.bfloat16 and self.use_tc and self.tc_variant != "tap" and self.fuse_conv_out and pk.w_tc is not None
+                and pk.Co % 8 != 0 and Cc % 64 == 0 and pk.k[2] <= 3 and T > tp):
+            # conv_out writes the reconstruction in torch's (B,C,T,H,W) layout itself and never computes the time_padding
+            # frames the reference drops afterwards (M:1642-1647)
+            return self.conv(x, pk, pad=(pk.k[0] - 1 - tp, pk.k[1] // 2, pk.k[2] // 2), out_spatial=(T - tp, H, W), out_cf=True), saved
+        return self.to_channels_first(self.conv(x, pk), t_crop=tp), saved
+
+    def encode_cl(self, video: torch.Tensor, first_frame: bool = True, cond=None):
+        """video (B,C,T,H,W) on device -> encoder output, channels-last.  Reference encode M:1523-1576."""
+        m = self.model
+        x, _ = self.conv_in_cl(video, first_frame)
         self._tap("conv_in", x)
         cond_e = self.cond_stem(cond, "enc") if (m.has_cond and cond is not None) else None     # M:1544-1548
         for i, st in enumerate(m.stages):
@@ -715,35 +770,14 @@ class Engine:
         return x
 
     def decode_cl(self, q: torch.Tensor, first_frame: bool = True, cond=None):
-        """quantized channels-last (B,T',H',W',C) -> video (B,3,T,H,W).  Reference decode M:1598-1649; the leading
-        time_padding frames are dropped only for clips that contain a first frame (M:1646-1647)."""
+        """quantized channels-last (B,T',H',W',C) -> video (B,3,T,H,W).  Reference decode M:1598-1649."""
         m = self.model
         x = q
         cond_e = self.cond_stem(cond, "dec") if (m.has_cond and cond is not None) else None     # M:1612-1616
         for j, st in enumerate(reversed(m.stages)):
             x = self._stage(x, st, f"dec{j}", decoder=True, cond_e=cond_e)
             self._tap(f"dec{j}", x)
-        pk = self._packs["conv_out"]
-        B, T, H, W, Cc = x.shape
-        tp = m.time_padding if first_frame else 0
-        if m.separate_first_frame_encoding and first_frame:
-            # M:1633-1639: conv_out_first_frame on frame `tp`, the causal conv_out on the frames after it, re-attached
-            first = self.conv(self.copy_frames(x, tp, 1), self._packs["conv_out_ff"])
-            out = self._new((B, T - tp, H, W, first.shape[-1]))
-            self.copy_frames(first, 0, 1, dst=out, dst_t0=0)
-            if T - tp > 1:
-                rest = self.causal_conv_padded(self.copy_frames(x, tp + 1, T - tp - 1), pk, m.conv_out.pad_mode)
-                self.copy_frames(rest, 0, T - tp - 1, dst=out, dst_t0=1)
-            return self.to_channels_first(out)
-        if m.conv_out.pad_mode != "constant":
-            return self.to_channels_first(self.causal_conv_padded(x, pk, m.conv_out.pad_mode), t_crop=tp)
-        if (self.dtype == torch.bfloat16 and self.use_tc and self.tc_variant != "tap" and self.fuse_conv_out and pk.w_tc is not None
-                and pk.Co % 8 != 0 and Cc % 64 == 0 and pk.k[2] <= 3 and T > tp):
-            # conv_out writes the reconstruction in torch's (B,C,T,H,W) layout itself and never computes the time_padding
-            # frames the reference drops afterwards (M:1642-1647)
-            return self.conv(x, pk, pad=(pk.k[0] - 1 - tp, pk.k[1] // 2, pk.k[2] // 2), out_spatial=(T - tp, H, W), out_cf=True)
-        x = self.conv(x, pk)
-        return self.to_channels_first(x, t_crop=tp)
+        return self.conv_out_cf(x, first_frame)[0]
 
     def quantize_cl(self, x, want_quantized=True, want_aux=False):
         """x channels-last -> (quantized channels-last | None, indices (B,T,H,W[,num_codebooks]), aux fp32 [N][D] | None)."""

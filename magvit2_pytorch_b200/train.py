@@ -26,8 +26,7 @@ from typing import Callable, Dict, List, Sequence
 import torch
 import torch.nn.functional as F
 
-from ._lib import ACT_ELU, check
-from .engine import _dt, _ptr
+from .engine import pack_conv, stage_modules
 
 
 # --------------------------------------------------------------------------------------------
@@ -273,7 +272,6 @@ class TrainRunner:
         gx = None
         own_dgrad = need_gx and self.own_dgrad and causal_default and tuple(stride) == (1, 1, 1) and not x_is_cf
         if own_dgrad:
-            from .engine import pack_conv
             wt = w5.detach().flip(2, 3, 4).transpose(0, 1).contiguous()          # (Ci, Co, kt, kh, kw): dgrad weights
             gx = self.eng.conv(g.contiguous(), pack_conv(wt, None, self.eng.dtype), pad=(0, ph, pw), out_spatial=tuple(x.shape[1:4]))
             self.own_dgrad_calls += 1
@@ -317,24 +315,10 @@ class TrainRunner:
         return gx.permute(0, 2, 3, 4, 1).contiguous()
 
     # ---- forward pieces (engine kernels) that record their backward
-    def _residual_unit(self, x, p, ru):
-        """ResidualUnit (M:930-944) unfused: both conv outputs and the SE gates are kept for the backward."""
-        eng, lib = self.eng, self.eng.lib
-        seq = ru.fn
-        c3m, c1m, se = seq[0].conv, seq[2], seq[4]
-        B, T, H, W, Cc = x.shape
-        F_, Pn = B * T, H * W
-        st, dt = eng._stream(), _dt(eng.dtype)
-        h = eng.conv(x, p["conv3"], act=ACT_ELU)
-        y = eng.conv(h, p["conv1"], act=ACT_ELU)
-        ws = eng._new((lib.mv2_se_workspace_bytes(F_, Pn, Cc) // 4,), torch.float32)
-        gates = eng._new((F_, Cc), torch.float32)
-        check(lib.mv2_se_pool(_ptr(y), dt, F_, Pn, Cc, _ptr(p["wk"]), p["bk"], _ptr(ws), st), "mv2_se_pool")
-        check(lib.mv2_se_gate(_ptr(ws), dt, F_, Pn, Cc, p["hidden"], _ptr(p["w1"]), _ptr(p["b1"]), _ptr(p["w2"]), _ptr(p["b2"]),
-                              _ptr(gates), st), "mv2_se_gate")
-        out = eng._new(x.shape)
-        check(lib.mv2_gate_residual(_ptr(y), _ptr(x), _ptr(gates), _ptr(out), dt, F_, Pn, Cc, st), "mv2_gate_residual")
-        eng.launches += 3
+    def _residual_unit(self, x, p, u):
+        """ResidualUnit (M:930-944) unfused: both conv outputs are kept for the backward."""
+        out, h, y = self.eng.residual_unit_unfused(x, p)
+        c3m, c1m, se = u["conv3"], u["conv1"], u["se"]
         k3 = tuple(c3m.weight.shape[2:])
 
         def bwd(g):
@@ -352,11 +336,12 @@ class TrainRunner:
         self.tape.append(lambda g: self._vjp(fn, x, params, g))
         return out
 
-    def _stage(self, x, st, key, mod, decoder, cond_e=None):
+    def _stage(self, x, st, key, parts, decoder, cond_e=None):
+        """One stage through the engine; `parts` = engine.stage_modules(...) of its layer module."""
         eng = self.eng
         P = eng._packs
-        B, T, H, W, Cc = x.shape
         if st.kind == "cond_residual":
+            mod = parts["unit"]
             side = "dec" if decoder else "enc"
             xin = x
             out = eng._stage(x, st, key, decoder=decoder, cond_e=cond_e)
@@ -371,12 +356,11 @@ class TrainRunner:
             self.tape.append(bwd)
             return out
         if st.kind == "residual":
-            units = list(mod) if st.nested else [mod]
-            for j, ru in enumerate(units):
-                x = self._residual_unit(x, P[f"{key}.{j}"], ru)
+            for j, u in enumerate(parts["units"]):
+                x = self._residual_unit(x, P[f"{key}.{j}"], u)
             return x
         if st.kind in ("compress_space", "compress_time") and not decoder:
-            conv = mod.conv
+            conv = parts["conv"]
             if st.kind == "compress_space":     # SpatialDownsample2x (M:770-780): Conv2d k3 s2 p1 per frame
                 k, stride, pad = (1, 3, 3), (1, 2, 2), (0, 1, 1)
             else:                               # TimeDownsample2x (M:796-807): F.pad (2, 0) + Conv1d k3 s2 per pixel
@@ -387,18 +371,17 @@ class TrainRunner:
             return out
         run = lambda t: eng._stage(t, st, key, decoder=decoder)       # noqa: E731
         if st.kind == "compress_space":
-            conv = mod.net[0]
+            conv = parts["conv"]
             return self._block(x, run, lambda t: _upsample_space(t, conv), list(conv.parameters()))
         if st.kind == "compress_time":
-            conv = mod.net[0]
+            conv = parts["conv"]
             return self._block(x, run, lambda t: _upsample_time(t, conv), list(conv.parameters()))
         if st.kind == "gateloop_time":
-            gl = mod.fn.fn
+            gl = parts["gateloop"]
             return self._block(x, run, lambda t: _gateloop_block(t, gl), list(gl.parameters()))
         if st.kind in ("attend_space", "attend_time", "linear_attend_space"):
             time_axis = st.kind == "attend_time"
-            at = mod[0].fn.fn if time_axis else mod[0].fn
-            ff = mod[1].fn.fn if time_axis else mod[1].fn
+            at, ff = parts["attn"], parts["ff"]
             if st.kind == "linear_attend_space":
                 x = self._block(x, lambda t: eng.linear_attention(t, P[key + ".attn"]), lambda t: _linear_attention_block(t, at),
                                 list(at.parameters()))
@@ -414,48 +397,28 @@ class TrainRunner:
         """-> (recon (B,C,T,H,W), aux_loss 0-d fp32); codes / the LFQ breakdown are left in .codes / .breakdown."""
         from .dist import LfqBatchEntropy
         m, eng = self.m, self.eng
-        P = eng._packs
         self.cond = cond
         ce_enc = eng.cond_stem(cond, "enc") if m.has_cond else None            # M:1544-1548 (Linear + SiLU stems)
         ce_dec = eng.cond_stem(cond, "dec") if m.has_cond else None            # M:1612-1616
         t_pad = m.time_padding if first_frame else 0
         cin, cout = m.conv_in.conv, m.conv_out.conv
         kin = tuple(cin.weight.shape[2:])
-        pin = P.get("conv_in_tc")
         sff = bool(m.separate_first_frame_encoding and first_frame)
         mode_in, mode_out = m.conv_in.pad_mode, m.conv_out.pad_mode
-        vid = video
-        if sff:
-            # M:1553-1561: the first frame through its own 2-D conv, frames 1.. through the causal conv_in on their own
-            Bv, _, Tv, Hv, Wv = video.shape
-            v_cl = eng.to_channels_last(video, 0)
-            first = eng.conv(eng.copy_frames(v_cl, 0, 1), P["conv_in_ff"])
-            x = eng._new((Bv, Tv + t_pad, Hv, Wv, first.shape[-1]))
-            eng.copy_frames(first, 0, 1, dst=x, dst_t0=t_pad, zero_front=True)
-            rest_in = eng.copy_frames(v_cl, 1, Tv - 1) if Tv > 1 else None
-            if Tv > 1:
-                rest = eng.causal_conv_padded(rest_in, P["conv_in"], mode_in)
-                eng.copy_frames(rest, 0, Tv - 1, dst=x, dst_t0=t_pad + 1)
-        elif mode_in != "constant":
-            padded_in = eng.to_channels_last(video, t_pad)               # time_padding zero frames first (M:1537), then the mode's pad
-            x = eng.causal_conv_padded(padded_in, P["conv_in"], mode_in)
-        elif eng.dtype == torch.bfloat16 and eng.use_tc and pin is not None:
-            x = eng.conv(eng.ingest_kwpack(video, t_pad, pin), pin, pad=(pin.k_tc[0] - 1, pin.k_tc[1] // 2, 0))
-        else:
-            x = eng.conv(eng.to_channels_last(video, t_pad), P["conv_in"])
+        x, saved_in = eng.conv_in_cl(video, first_frame)
 
         def bwd_conv_in(g):     # the video needs no gradient: weight / bias only
-            v = (vid.float() / 255. if vid.dtype == torch.uint8 else vid).to(eng.dtype)
+            v = (video.float() / 255. if video.dtype == torch.uint8 else video).to(eng.dtype)
             if sff:
                 ff = m.conv_in_first_frame
                 kff = (1,) + tuple(ff.weight.shape[2:])
                 self._conv_bwd(g[:, t_pad:t_pad + 1].contiguous(), v[:, :, 0:1], ff.weight, ff.bias, kff, pad=(0, kff[1] // 2, kff[2] // 2),
                                need_gx=False, x_is_cf=True)
                 if v.shape[2] > 1:
-                    self._conv_bwd_padmode(g[:, t_pad + 1:].contiguous(), rest_in, cin.weight, cin.bias, kin, mode_in, need_gx=False)
+                    self._conv_bwd_padmode(g[:, t_pad + 1:].contiguous(), saved_in["rest_in"], cin.weight, cin.bias, kin, mode_in, need_gx=False)
                 return None
             if mode_in != "constant":
-                self._conv_bwd_padmode(g, padded_in, cin.weight, cin.bias, kin, mode_in, need_gx=False)
+                self._conv_bwd_padmode(g, saved_in["padded_in"], cin.weight, cin.bias, kin, mode_in, need_gx=False)
                 return None
             self._conv_bwd(g, v, cin.weight, cin.bias, kin, pad=(t_pad + kin[0] - 1, kin[1] // 2, kin[2] // 2),
                            need_gx=False, x_is_cf=True)
@@ -463,7 +426,7 @@ class TrainRunner:
 
         self.tape.append(bwd_conv_in)
         for i, st in enumerate(m.stages):
-            x = self._stage(x, st, f"enc{i}", m.encoder_layers[i], decoder=False, cond_e=ce_enc)
+            x = self._stage(x, st, f"enc{i}", stage_modules(st, m.encoder_layers[i], False), decoder=False, cond_e=ce_enc)
 
         qz = m.quantizers
         if m.use_fsq:
@@ -487,22 +450,10 @@ class TrainRunner:
 
         x = q
         for j, st in enumerate(reversed(m.stages)):
-            x = self._stage(x, st, f"dec{j}", m.decoder_layers[j], decoder=True, cond_e=ce_dec)
+            x = self._stage(x, st, f"dec{j}", stage_modules(st, m.decoder_layers[j], True), decoder=True, cond_e=ce_dec)
         xo = x
         kout = tuple(cout.weight.shape[2:])
-        if sff:
-            # M:1633-1639: conv_out_first_frame on frame t_pad, the causal conv_out on the frames after it, re-attached
-            Bx, Tx, Hx, Wx, _ = x.shape
-            first = eng.conv(eng.copy_frames(x, t_pad, 1), P["conv_out_ff"])
-            y = eng._new((Bx, Tx - t_pad, Hx, Wx, first.shape[-1]))
-            eng.copy_frames(first, 0, 1, dst=y, dst_t0=0)
-            rest_out = eng.copy_frames(x, t_pad + 1, Tx - t_pad - 1) if Tx - t_pad > 1 else None
-            if Tx - t_pad > 1:
-                eng.copy_frames(eng.causal_conv_padded(rest_out, P["conv_out"], mode_out), 0, Tx - t_pad - 1, dst=y, dst_t0=1)
-            recon = eng.to_channels_first(y)
-        else:
-            y = eng.causal_conv_padded(x, P["conv_out"], mode_out)
-            recon = eng.to_channels_first(y, t_crop=t_pad)
+        recon, saved_out = eng.conv_out_cf(x, first_frame)
 
         def bwd_conv_out(g_recon):    # (B,C,T,H,W) -> channels-last with zero gradient on the cropped time_padding frames
             g = g_recon.permute(0, 2, 3, 4, 1)
@@ -513,7 +464,7 @@ class TrainRunner:
                 gx[:, t_pad:t_pad + 1] = self._conv_bwd(g[:, 0:1].contiguous(), xo[:, t_pad:t_pad + 1].contiguous(), off.weight, off.bias, kff,
                                                         pad=(0, kff[1] // 2, kff[2] // 2))
                 if xo.shape[1] - t_pad > 1:
-                    gx[:, t_pad + 1:] = self._conv_bwd_padmode(g[:, 1:].contiguous(), rest_out, cout.weight, cout.bias, kout, mode_out)
+                    gx[:, t_pad + 1:] = self._conv_bwd_padmode(g[:, 1:].contiguous(), saved_out["rest_out"], cout.weight, cout.bias, kout, mode_out)
                 return gx
             if t_pad:
                 g = F.pad(g, (0, 0, 0, 0, 0, 0, t_pad, 0))
